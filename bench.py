@@ -58,8 +58,37 @@ def parse():
     ap.add_argument("--clip", type=float, default=0.0, help="gradient_clipping (both arms)")
     ap.add_argument("--gas", type=int, default=1, help="gradient_accumulation_steps (both arms); a timed step = one "
                     "optimizer step = GAS micro-batches")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="b200 arm: after the timed steps, write what the last timed step computed to DIR/<name>.npy")
     ap.add_argument("--local_rank", type=int, default=0)
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.dump_outputs and args.steps + args.warmup < 1:
+        ap.error("--dump-outputs needs at least one step (--steps or --warmup) to take its outputs from")
+    return args
+
+
+def dump_outputs(torch, engine, losses, out_dir, rank, max_params=3, max_numel=1 << 26, sample=1 << 20):
+    """What one training step hands its caller: the loss of each micro-batch, and the updated model.  The model is
+    represented by the fp32 master weights of ``max_params`` weight matrices (first, middle and last of those with at
+    most ``max_numel`` elements), each as a fixed seeded sample of ``sample`` elements; float32, about 12 MB in all.
+    Collective under ZeRO-3: every rank calls it, rank 0 writes."""
+    import numpy as np
+    from deepspeed_b200.utils import safe_get_full_fp32_param
+    arrays = {"loss": torch.stack([l.float().reshape(()) for l in losses]).cpu()}
+    named = [(n, p) for n, p in engine.module.named_parameters()
+             if len(getattr(p, "ds_shape", p.shape)) == 2 and int(getattr(p, "ds_numel", p.numel())) <= max_numel]
+    picks = sorted({round(i * (len(named) - 1) / max(1, max_params - 1)) for i in range(max_params)}) if named else []
+    for i in picks:
+        name, p = named[i]
+        full = safe_get_full_fp32_param(p).reshape(-1)
+        if full.numel() > sample:
+            idx = torch.randint(0, full.numel(), (sample, ), generator=torch.Generator().manual_seed(i))
+            full = full[idx.to(full.device)]
+        arrays[f"param.{name}"] = full.float().cpu()
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, f"{name}.npy"), a.numpy().astype(np.float32))
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -306,6 +335,7 @@ def run_b200(args):
     loss_host = torch.zeros(1, dtype=torch.float32).pin_memory()
 
     gas = args.gas
+    last_losses = [None] * gas  # the micro-batch losses of the latest step, for --dump-outputs
 
     def fwd(ids):
         return engine(input_ids=ids, labels=ids).loss if hf else engine(ids, labels=ids)
@@ -315,6 +345,7 @@ def run_b200(args):
             loss = fwd(dev[(i * gas + k) % n_batches])
             engine.backward(loss)
             engine.step()
+            last_losses[k] = loss.detach()
 
     def step_e2e(i):
         for k in range(gas):
@@ -322,6 +353,7 @@ def run_b200(args):
             loss = fwd(ids)
             engine.backward(loss)
             engine.step()
+            last_losses[k] = loss.detach()
         loss_host.copy_(loss.detach().float().reshape(1), non_blocking=False)  # D2H read of the result
 
     try:
@@ -348,6 +380,8 @@ def run_b200(args):
     launches = native.launch_count - l0
     t_e2e = timed_loop(torch, ds.comm, world, args.steps, step_e2e)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(torch, engine, last_losses, args.dump_outputs, rank)
     # exposed (non-overlapped) communication: 2 extra, untimed-for-throughput steps with every compute-stream
     # wait on a collective bracketed by CUDA events (the bracket holds no kernels => elapsed == stall)
     exposed = None

@@ -122,19 +122,6 @@ def test_random_ltd_wrapper_and_scheduler():
     assert all(".random_ltd_layer" not in k for k in save_without_random_ltd(model))
 
 
-def _load_reference_indexed_dataset():
-    import importlib.util
-    import os
-    for root in ("/root/reference/deepspeed", os.path.join(os.path.dirname(__file__), "..", "..", "baseline", "_ref", "deepspeed")):
-        f = os.path.join(root, "runtime", "data_pipeline", "data_sampling", "indexed_dataset.py")
-        if os.path.exists(f):
-            spec = importlib.util.spec_from_file_location("_ref_indexed_dataset", f)
-            mod = importlib.util.module_from_spec(spec)
-            spec.loader.exec_module(mod)
-            return mod
-    return None
-
-
 def test_indexed_dataset_formats_and_interop(tmp_path):
     import numpy as np
     import torch
@@ -167,22 +154,18 @@ def test_indexed_dataset_formats_and_interop(tmp_path):
     assert I.code(np.int64) == 5 and I.code(torch.int16) == 3 and I.create_doc_idx([3, 0, 2, 0]) == [0, 2, 4]
     p, tot = I.get_pointers_with_total([2, 3, 4], 4, np.int64)
     assert p.tolist() == [0, 8, 20] and tot == 36
-    # --- cross-check both directions against the reference implementation when its source is around
-    R = _load_reference_indexed_dataset()
-    if R is None:
-        return
-    rds = R.MMapIndexedDataset(meg, skip_warmup=True)
-    assert len(rds) == 3 and all(np.array_equal(rds[i], s) for i, s in enumerate(samples))
-    assert rds.doc_idx.tolist() == ds.doc_idx.tolist()
-    theirs = str(tmp_path / "theirs")
-    rb = R.MMapIndexedDatasetBuilder(R.data_file_path(theirs), dtype=np.int32)
-    for s in samples:
-        rb.add_item(torch.from_numpy(s))
-        rb.end_document()
-    rb.finalize(R.index_file_path(theirs))
-    mine = I.MMapIndexedDataset(theirs)
+    # --- both directions against upstream DeepSpeed's indexed_dataset.py, through files its builders wrote for the same
+    # samples (tests/golden/indexed_dataset, regenerate: scripts/make_reference_golden.py)
+    import os
+    golden = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "golden", "indexed_dataset")
+    for prefix, theirs in ((meg, "mmap_uint16"), (pre, "legacy_int32")):  # upstream reads ours: the bytes are its own
+        for ext in (".bin", ".idx"):
+            with open(prefix + ext, "rb") as a, open(os.path.join(golden, theirs + ext), "rb") as b:
+                assert a.read() == b.read(), theirs + ext
+    mine = I.MMapIndexedDataset(os.path.join(golden, "mmap_int32"))
     assert mine.dtype == np.int32 and all(np.array_equal(mine[i], s) for i, s in enumerate(samples))
-    rl = R.IndexedDataset(pre)
+    assert mine.doc_idx.tolist() == ds.doc_idx.tolist()
+    rl = I.make_dataset(os.path.join(golden, "legacy_int32"), "lazy")
     assert all(np.array_equal(rl[i], s) for i, s in enumerate(samples))
 
 
